@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            our CUDA path (libdsin_b200)
   python bench.py --impl reference ...                      the reference arithmetic on host cores
+  python bench.py ... --dump-outputs DIR                    also write the last timed step's outputs to DIR/*.npy
 
 A "step" is one AE.siNet_get_reconstructed-equivalent pass (AE(y), AE(x), bpp, SI-Finder, SI-Net;
 /root/reference/src/AE.py:132-148) over one batch of synthetic 320x1224 pairs.
@@ -51,6 +52,38 @@ def set_geometry(hw):
 
 def log(*a):
     print(*a, file=sys.stderr, flush=True)
+
+
+def load_library():
+    """libdsin_b200 as __graft_entry__.build() left it.  Nothing is compiled here: the tree may be read-only."""
+    import __graft_entry__ as g
+    if g._stale():
+        sys.exit("bench.py: dsin_b200/libdsin_b200.so is missing or older than its sources; "
+                 "run `python -c 'import __graft_entry__ as g; g.build()'` first")
+    from dsin_b200 import _lib
+    _lib.load()
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, parts):
+    """Writes what the last timed step returned, one dict of CUDA tensors per micro-batch, as path/<name>.npy:
+    float64 outputs as float64, all others as float32 (the integer outputs are small enough to be exact).  Each output
+    is concatenated over the micro-batches; one with more elements than its share of DUMP_BYTES is written as a
+    sample of its flattened elements, at indices drawn with a fixed seed and kept in ascending order, so that two
+    runs with the same arguments write the same elements."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    names = sorted(parts[0])
+    cap = DUMP_BYTES // (8 * len(names))  # elements per output, even if all are float64
+    for name in names:
+        t = torch.cat([p[name] for p in parts])
+        if t.numel() > cap:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), cap, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        t = t.to(torch.float64 if t.dtype == torch.float64 else torch.float32)
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy())
 
 
 def peaks():
@@ -186,7 +219,7 @@ def run_reference(args, rank):
     for i in range(1 if args.warmup >= 1 else 0):  # one warm-up pair is enough on CPU
         oracle_seconds_per_pair(1, seed=50 + i)
     times = []
-    steps = max(1, min(args.steps, 5))  # bounded sample: <= 5 pairs (~10 s each)
+    steps = args.steps
     for i in range(steps):
         s, cores = oracle_seconds_per_pair(1, seed=i)
         times.append(s)
@@ -226,10 +259,8 @@ def build_ae(device_index, residual_gamma=0.25, precision=None):
 def run_ours(args, rank, world, local_rank):
     import torch
     import torch.distributed as dist
-    import __graft_entry__ as g
     torch.cuda.set_device(local_rank)
-    if rank == 0:
-        g.build()
+    load_library()
     if world > 1:
         # NCCL writes its version / debug lines to the C-level stdout when NCCL_DEBUG is set in the environment:
         # point fd 1 at stderr while the communicator comes up, so that stdout carries the one JSON line only
@@ -243,8 +274,6 @@ def run_ours(args, rank, world, local_rank):
         finally:
             os.dup2(saved_fd, 1)
             os.close(saved_fd)
-    if rank != 0:
-        g.build()  # no-op: rank 0 has built; this only loads/validates the library
     from dsin_b200 import ops, precision, synth
     from dsin_b200.dist import gather_metrics, shard_range
     pk = peaks()
@@ -295,6 +324,8 @@ def run_ours(args, rank, world, local_rank):
     launches_per_step = ops.launch_count() - l0
 
     bits_parts = []
+    last_step = []  # --dump-outputs: each micro-batch's outputs in the last timed step, less "dec" = [y_dec; x_dec]
+    dump = args.dump_outputs is not None and rank == 0
 
     def step_graph(i, keep=False):
         for j, m in enumerate(micro):
@@ -302,6 +333,8 @@ def run_ours(args, rank, world, local_rank):
             out = ae.replay_device(xd[:m], yd[:m])
             if keep:
                 bits_parts.append(out["bits_sum"].clone())  # graph outputs are static buffers
+            if keep and dump and i == args.steps - 1:
+                last_step.append({k: v.clone() for k, v in out.items() if torch.is_tensor(v) and k != "dec"})
         return out
 
     for i in range(args.warmup):
@@ -322,6 +355,9 @@ def run_ours(args, rank, world, local_rank):
     ms = e0.elapsed_time(e1)
     launches = launches_per_step * args.steps
     clocks = sampler.stop() if rank == 0 else None
+    if dump:
+        dump_outputs(args.dump_outputs, last_step)
+        del last_step[:]
     bits_total = float(sum(float(b.sum().item()) for b in bits_parts))
     npix_total = n_local * args.steps * H * W
 
@@ -487,9 +523,8 @@ def run_ours(args, rank, world, local_rank):
 def run_sif_only(args, rank, world, local_rank):
     """BASELINE configs[2]: SI-Finder (prepare + match + gather) in isolation on device-resident inputs."""
     import torch
-    import __graft_entry__ as g
     torch.cuda.set_device(local_rank)
-    g.build()
+    load_library()
     from dsin_b200 import ops, synth
     from dsin_b200.siFinder import match_images
     pk = peaks()
@@ -539,9 +574,8 @@ def run_enc_only(args, rank, world, local_rank):
     """BASELINE configs[3]: encoder + quantiser + probability model (the sender's rate path: symbols and bpp) on
     batch 64 of 320x960 crops, device-resident inputs; src/AE.py:50-53,85-87."""
     import torch
-    import __graft_entry__ as g
     torch.cuda.set_device(local_rank)
-    g.build()
+    load_library()
     if not args.hw:
         set_geometry("320x960")
     from dsin_b200 import ops, precision, synth
@@ -610,9 +644,8 @@ def run_enc_only(args, rank, world, local_rank):
 def run_codec(args, rank, world, local_rank):
     """SURVEY 8f N3: PC1 entropy coder (range coder driven by the probability model) on the symbols of one batch."""
     import torch
-    import __graft_entry__ as g
     torch.cuda.set_device(local_rank)
-    g.build()
+    load_library()
     from dsin_b200 import ops, synth
     B = args.batch
     ae = build_ae(local_rank)
@@ -669,9 +702,8 @@ def run_roundtrip(args, rank, world, local_rank):
     """Sender and receiver with real bitstreams through the public numpy API: compress(x) -> bytes;
     decompress(bytes, y) -> y_dec, y_syn, x_dec, x_with_si (host buffers on both sides)."""
     import torch
-    import __graft_entry__ as g
     torch.cuda.set_device(local_rank)
-    g.build()
+    load_library()
     from dsin_b200 import synth
     B = args.batch
     ae = build_ae(local_rank)
@@ -732,7 +764,14 @@ def main():
     ap.add_argument("--workload", default="full", choices=["full", "sif", "enc", "codec", "roundtrip"],
                     help="full = configs[4] / configs[1]; sif = configs[2] (SI-Finder in isolation, --batch 32); "
                          "enc = configs[3] (encoder + quantiser + probclass on 320x960 crops, --batch 64)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="--workload full: after the timed steps, write what the last one returned (rank 0's pairs) "
+                         "to DIR/<name>.npy, at most 64 MB in all; the copies of that step's outputs are timed with it")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and (args.impl != "ours" or args.workload != "full"):
+        ap.error("--dump-outputs writes the outputs of --impl ours --workload full")
     if args.hw:
         set_geometry(args.hw)
     rank = int(os.environ.get("RANK", "0"))

@@ -1,6 +1,7 @@
 """Generates tests/golden/*.npz from the parts of the reference that run in this container.
 
-Run here (needs /root/reference):  python tests/golden/make_golden.py
+Run from the repository root with a checkout of the reference (ayziksha/DSIN):
+    python tests/golden/make_golden.py <path of the DSIN checkout>
   * mask_golden.npz   - AE.create_gaussian_masks (src/AE.py:193-220), extracted with ``ast``
                         and executed with a stub ``self`` (pure numpy).
   * msssim_golden.npz - ms_ssim_np_imgcomp.MultiScaleSSIM / utils.msssim_x_vs_rec call forms
@@ -12,6 +13,7 @@ Run here (needs /root/reference):  python tests/golden/make_golden.py
                         helpers (:371-393), AE.normalize / denormalize / get_mean_var (src/AE.py:222-250), and the
                         host helpers readfiles (src/DataProvider.py:96-100), l1_x_vs_rec and save_test_imgs_fn
                         (src/utils.py:82-111).
+  * run_configs_golden.json - what src/run_configs/{ae,pc}_run_configs parse to (repr of every value).
   * tf_pieces_golden.npz - reference functions whose bodies are elementwise / shape TensorFlow ops only, extracted with
                         ``ast`` and executed under a small numpy stand-in for those ops (``_make_tf`` / ``_T`` below: tile,
                         expand_dims, split, concat, sigmoid, softmax, argmax, one_hot, reduce_sum, ... each following the
@@ -24,13 +26,14 @@ Run here (needs /root/reference):  python tests/golden/make_golden.py
 Nothing from the reference is copied into the repo; only its numeric outputs are stored.
 """
 import ast
+import json
 import os
 import sys
 import types
 
 import numpy as np
 
-REF = "/root/reference/src"
+REF = None  # src/ of the DSIN checkout named on the command line
 OUT = os.path.dirname(os.path.abspath(__file__))
 
 
@@ -336,12 +339,26 @@ def make_loss_pieces():
     np.savez_compressed(os.path.join(OUT, "loss_pieces_golden.npz"), **out)
 
 
+def make_configs():
+    sys.path.insert(0, os.path.dirname(os.path.dirname(OUT)))
+    from dsin_b200 import config_parser
+    out = {}
+    for name in ("ae_run_configs", "pc_run_configs"):
+        cfg, _ = config_parser.parse(os.path.join(REF, "run_configs", name))
+        out[name] = {k: repr(v) for k, v in cfg.all_params_and_values()}
+    with open(os.path.join(OUT, "run_configs_golden.json"), "w") as f:
+        json.dump(out, f, indent=1, sort_keys=True)
+        f.write("\n")
+
+
 if __name__ == "__main__":
+    REF = os.path.join(sys.argv[1], "src")
+    make_configs()
     make_loss_pieces()
     make_masks()
     make_msssim()
     make_model_pieces()
     make_tf_pieces()
     for f in ("mask_golden.npz", "msssim_golden.npz", "model_pieces_golden.npz", "tf_pieces_golden.npz",
-              "loss_pieces_golden.npz"):
+              "loss_pieces_golden.npz", "run_configs_golden.json"):
         print(f, os.path.getsize(os.path.join(OUT, f)))

@@ -1,8 +1,11 @@
-"""bench.py's JSON contract, checked on CPU through the reference arm at a reduced geometry."""
+"""bench.py's JSON contract, checked on CPU through the reference arm at a reduced geometry; --dump-outputs on the GPU."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -31,3 +34,27 @@ def test_non_zero_ranks_of_reference_arm_exit_quietly():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1",
                           "--warmup", "0", "--hw", "80x144"], capture_output=True, text=True, env=env, timeout=120, cwd=ROOT)
     assert out.returncode == 0 and out.stdout.strip() == ""
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_same_for_the_same_arguments(tmp_path):
+    """--dump-outputs: two runs with the same arguments write the same float32 / float64 arrays, 64 MB at most, and the
+    JSON line reports the requested number of timed steps.  6 pairs per step: every output is small enough to be
+    written whole, in its own shape."""
+    dumps = []
+    for run in ("a", "b"):
+        d = tmp_path / run
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "1", "--hw",
+                              "80x144", "--global-batch", "6", "--micro-batch", "4", "--no-cpu-baseline",
+                              "--dump-outputs", str(d)], capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert out.returncode == 0, out.stderr[-2000:]
+        lines = [l for l in out.stdout.splitlines() if l.startswith("{")]
+        assert len(lines) == 1 and json.loads(lines[0])["steps"] == 2
+        dumps.append({f: np.load(d / f) for f in os.listdir(d)})
+    a, b = dumps
+    assert {"y_dec.npy", "y_syn.npy", "x_dec.npy", "x_with_si.npy", "symbols.npy", "bits_sum.npy", "row.npy"} <= set(a)
+    assert sorted(a) == sorted(b) and sum(v.nbytes for v in a.values()) <= 64 << 20
+    assert a["x_with_si.npy"].shape == (6, 3, 80, 144) and a["row.npy"].shape[0] == 6
+    for k in a:
+        assert a[k].dtype in (np.float32, np.float64), k
+        assert np.array_equal(a[k], b[k]), k

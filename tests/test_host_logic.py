@@ -1,4 +1,5 @@
 """Host-side logic that runs without a GPU: config parser, synthetic generators, weight naming."""
+import json
 import os
 
 import numpy as np
@@ -22,14 +23,14 @@ def test_parse_shipped_configs():
     assert pc.use_centers_for_padding is True and pc.regularization_factor is None
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/src/run_configs/ae_run_configs"), reason="reference absent")
-def test_parse_reference_config_files_verbatim():
-    ae, _ = config_parser.parse("/root/reference/src/run_configs/ae_run_configs")
-    mine, _ = config_parser.parse(os.path.join(ROOT, "dsin_b200", "run_configs", "ae_run_configs"))
-    assert dict(ae.all_params_and_values()) == dict(mine.all_params_and_values())
-    pc, _ = config_parser.parse("/root/reference/src/run_configs/pc_run_configs")
-    minepc, _ = config_parser.parse(os.path.join(ROOT, "dsin_b200", "run_configs", "pc_run_configs"))
-    assert dict(pc.all_params_and_values()) == dict(minepc.all_params_and_values())
+def test_parse_reference_config_files_verbatim(golden_dir):
+    """The shipped run configs parse to exactly what the reference's src/run_configs parse to (repr of every value,
+    stored by tests/golden/make_golden.py)."""
+    with open(os.path.join(golden_dir, "run_configs_golden.json")) as f:
+        ref = json.load(f)
+    for name in ("ae_run_configs", "pc_run_configs"):
+        mine, _ = config_parser.parse(os.path.join(ROOT, "dsin_b200", "run_configs", name))
+        assert {k: repr(v) for k, v in mine.all_params_and_values()} == ref[name]
 
 
 def test_constraint_violation_and_bad_lines():
