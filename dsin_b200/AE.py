@@ -27,7 +27,7 @@ from . import precision as precision_policy
 from . import probclass_imgcomp as probclass
 from . import synth
 from . import tf_checkpoint
-from .siFinder import GaussianPrior
+from .siFinder import GaussianPrior, uses_l2
 
 
 def _host_copy(dst, a):
@@ -176,7 +176,7 @@ class AE(object):
         xs, ys = self._stage(x, "x"), self._stage(y, "y")
         if self.use_cuda_graph:
             out = self.replay_device(xs, ys)
-            xd = self._graphs[(xs.shape[0], xs.shape[2], xs.shape[3])]["x"]
+            xd = self._graph_state(xs.shape[0], xs.shape[2], xs.shape[3])["x"]
         else:
             xd = xs.to(torch.float32)
             out = self.reconstruct_device(xd, ys.to(torch.float32))
@@ -298,8 +298,9 @@ class AE(object):
     def _graph_state(self, B, H, W):
         """Capture (once per shape) the three segments of the inference step -- AE(y) + AE(x) + bit cost, SI-Finder,
         SI-Net -- as CUDA graphs over static buffers (segments, so that each segment's outputs can be copied to the host
-        while the next one runs)."""
-        key = (B, H, W)
+        while the next one runs).  The SI-Finder's matching mode is part of the key: switching ae_config.use_L2andLAB
+        on a live AE captures the other mode's graphs instead of replaying these."""
+        key = (B, H, W, uses_l2(self.ae_config))
         st = self._graphs.get(key)
         if st is not None:
             return st

@@ -57,6 +57,9 @@ SIGNATURES = {
     "dsin_sif_prepare": (_I, [_P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P]),
     "dsin_sif_workspace_bytes": (_I64, [_I, _I, _I, _I, _I, _I]),
     "dsin_sif_match": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P]),
+    "dsin_sif_prepare_lab": (_I, [_P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P]),
+    "dsin_sif_match_l2": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P]),
+    "dsin_sif_work_count_offset": (_I64, [_P, _I, _I, _I, _I, _I]),
     "dsin_msssim_workspace_bytes": (_I64, [_I, _I, _I, _I, _I]),
     "dsin_msssim": (_I, [_P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _P]),
     "dsin_validation_terms": (_I, [_P, _P, _P, _P, _P, _P, _I, _I64, _I64, _I, _P, _P]),

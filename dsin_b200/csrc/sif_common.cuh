@@ -1,7 +1,16 @@
-// Shared SI-Finder device helpers: the reference's Pearson algebra in literal fp32, the exact
+// Shared SI-Finder device helpers: the reference's Pearson and L2 algebra in literal fp32, the exact
 // Gaussian prior, and the packed (score, first-index) key used for argmax reductions.
 #pragma once
 #include "common.cuh"
+
+// Matching metric (ae_config.use_L2andLAB, src/siFinder.py:13-17,28-31,102-103).  The L2 path ranks the NEGATED
+// masked distance, so every argmax reduction, the packed keys and the first-index tie-break serve tf.argmin unchanged.
+enum SifMetric { SIF_PEARSON = 0, SIF_L2 = 1 };
+
+// src/siFinder.py:103 (L2 branch): out = sum_x_square - 2*xy + sum_y_square, evaluated (sx2 - 2*xy) + sy2 in fp32.
+__device__ __forceinline__ float sif_l2(float xy, float sx2, float sy2) {
+  return __fadd_rn(__fsub_rn(sx2, __fmul_rn(2.f, xy)), sy2);
+}
 
 // src/siFinder.py:114-133, evaluated left to right in fp32 without FMA contraction.
 //   num = xy - y_mean*sum_x - sum_y*x_mean + n*(y_mean*x_mean);  out = num / sqrt(den_y*den_x)
@@ -46,6 +55,7 @@ __device__ __forceinline__ void sif_unpack(unsigned long long k, float* s, unsig
 
 // tcgen05 coarse scorer + exact rescoring (sif_tc.cu)
 int64_t sif_tc_workspace_bytes(int n, int hh, int ww, int ph, int pw, int method);
+int64_t sif_tc_work_count_offset(const void* ws, int n, int hh, int ww, int ph, int pw);
 int sif_tc_match(dsin_handle_t h, const float* q, const float* r, const float* pstat, const float* ystat,
-                 int n, int hh, int ww, int ph, int pw, int use_mask, unsigned long long* keys, void* ws,
+                 int n, int hh, int ww, int ph, int pw, int use_mask, int metric, unsigned long long* keys, void* ws,
                  cudaStream_t st);

@@ -2,6 +2,8 @@
 // src/siFull_img.py:5-68, src/siFinder.py:7-53,56-73,76-135,138-154, src/AE.py:193-220.
 // The (h,w,P) correlation map (1.18 GB at 320x1224) and the Gaussian prior are never stored:
 // scores are produced tile by tile and reduced to a packed (score, index) key per patch.
+#include <type_traits>
+
 #include "common.cuh"
 #include "sif_common.cuh"
 
@@ -18,6 +20,42 @@ __device__ __forceinline__ void sif_transform(const float* __restrict__ px, floa
   out[2] = __fmul_rn(0.5f, __fadd_rn(R, B));
 }
 
+// rgb_to_lab (src/siFinder.py:157-195) on the RAW 0..255 pixel values (the L2 branch skips the normalisation,
+// :13-17), so the results lie far outside the usual CIELAB ranges (white: L ~ 9342).  Python scalars are float32
+// constants, as TF makes them.  `** 2.4` and `** (1/3)` are pow(x, 2.4f) and pow(x, 0.333333343f), evaluated in
+// fp64 and rounded once to fp32.  The 0/1-mask blends (:163-165,182-184) are branch selects: the inputs are finite
+// and >= 0, so both forms give the same bits.  The two 3x3 matmuls have no pinned summation order in TF; they are
+// defined here as left to right in fp32 without FMA (the oracle does the same).
+__device__ __forceinline__ float sif_lab_f(float t) {  // xyz_to_cielab's piecewise f
+  const float eps3 = 0.00885645207f, c3e2 = 0.12841855f, c429 = 0.137931034f;  // (6/29)^3, 3(6/29)^2, 4/29
+  return t <= eps3 ? __fadd_rn(__fdiv_rn(t, c3e2), c429) : (float)pow((double)t, (double)0.333333343f);
+}
+
+__device__ __forceinline__ void sif_lab(const float* __restrict__ px, float* out) {
+  float lin[3];
+#pragma unroll
+  for (int c = 0; c < 3; ++c) {
+    const float v = px[c];
+    lin[c] = v <= 0.04045f ? __fdiv_rn(v, 12.92f)
+                           : (float)pow((double)__fdiv_rn(__fadd_rn(v, 0.055f), 1.055f), (double)2.4f);
+  }
+  // rows R, G, B of rgb_to_xyz; columns X, Y, Z
+  const float X = __fadd_rn(__fadd_rn(__fmul_rn(lin[0], 0.412453f), __fmul_rn(lin[1], 0.357580f)),
+                            __fmul_rn(lin[2], 0.180423f));
+  const float Y = __fadd_rn(__fadd_rn(__fmul_rn(lin[0], 0.212671f), __fmul_rn(lin[1], 0.715160f)),
+                            __fmul_rn(lin[2], 0.072169f));
+  const float Z = __fadd_rn(__fadd_rn(__fmul_rn(lin[0], 0.019334f), __fmul_rn(lin[1], 0.119193f)),
+                            __fmul_rn(lin[2], 0.950227f));
+  const float fx = sif_lab_f(__fmul_rn(X, 1.05212653f));  // float32(1/0.950456)
+  const float fy = sif_lab_f(__fmul_rn(Y, 1.0f));
+  const float fz = sif_lab_f(__fmul_rn(Z, 0.918481112f));  // float32(1/1.088754)
+  // fxfyfz_to_lab, left to right, + [-16, 0, 0]
+  out[0] = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(fx, 0.f), __fmul_rn(fy, 116.f)), __fmul_rn(fz, 0.f)), -16.f);
+  out[1] = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(fx, 500.f), __fmul_rn(fy, -500.f)), __fmul_rn(fz, 0.f)), 0.f);
+  out[2] = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(fx, 0.f), __fmul_rn(fy, 200.f)), __fmul_rn(fz, -200.f)), 0.f);
+}
+
+template <int METRIC>
 __global__ void sif_transform_kernel(const float* __restrict__ xdec, const float* __restrict__ ydec,
                                      float* __restrict__ q, float* __restrict__ r, int n, int hh, int ww,
                                      int ph, int pw) {
@@ -25,11 +63,13 @@ __global__ void sif_transform_kernel(const float* __restrict__ xdec, const float
   int64_t npix = (int64_t)n * hh * ww;
   if (idx >= npix) return;
   float t[3];
-  sif_transform(ydec + idx * 3, t);
+  if constexpr (METRIC == SIF_L2) sif_lab(ydec + idx * 3, t);
+  else sif_transform(ydec + idx * 3, t);
   r[idx * 3 + 0] = t[0];
   r[idx * 3 + 1] = t[1];
   r[idx * 3 + 2] = t[2];
-  sif_transform(xdec + idx * 3, t);
+  if constexpr (METRIC == SIF_L2) sif_lab(xdec + idx * 3, t);
+  else sif_transform(xdec + idx * 3, t);
   int x = (int)(idx % ww);
   int64_t tt = idx / ww;
   int y = (int)(tt % hh);
@@ -115,10 +155,15 @@ __global__ void sif_ystat_kernel(const double2* __restrict__ hs, float* __restri
 }
 
 // ---------------------------------------------------------------------------------------------
-// K6 method 0: fp32 scoring of every (position, patch) on CUDA cores
+// K6 method 0: scoring of every (position, patch) on CUDA cores
 // tile = 64 positions of one correlation row x 64 patches; K loop over the ph patch rows.
+// Pearson accumulates the dot product in fp32.  L2 accumulates it in fp64 (exact products), rounded once to fp32 as
+// the oracle does: a ~1e10 fp32 sum of 1440 LAB products is off by far more than the gaps between distances.
 // ---------------------------------------------------------------------------------------------
-template <int PW>
+__device__ __forceinline__ float sif_mac(float a, float b, float c) { return fmaf(a, b, c); }
+__device__ __forceinline__ double sif_mac(float a, float b, double c) { return fma((double)a, (double)b, c); }
+
+template <int PW, int METRIC>
 __global__ void __launch_bounds__(256) sif_score_simt_kernel(const float* __restrict__ q,
                                                              const float* __restrict__ r,
                                                              const float* __restrict__ pstat,
@@ -139,11 +184,12 @@ __global__ void __launch_bounds__(256) sif_score_simt_kernel(const float* __rest
   const int tid = threadIdx.x, ty = tid / 16, tx = tid % 16;
   const int kdim = ph * KROW;
 
-  float acc[4][4];
+  using Acc = typename std::conditional<METRIC == SIF_L2, double, float>::type;
+  Acc acc[4][4];
 #pragma unroll
   for (int a = 0; a < 4; ++a)
 #pragma unroll
-    for (int b = 0; b < 4; ++b) acc[a][b] = 0.f;
+    for (int b = 0; b < 4; ++b) acc[a][b] = 0;
 
   for (int dy = 0; dy < ph; ++dy) {
     const float* rrow = r + (((int64_t)img * hh + i + dy) * ww + j0) * 3;
@@ -162,19 +208,19 @@ __global__ void __launch_bounds__(256) sif_score_simt_kernel(const float* __rest
       float a1 = s_r[(ty * 4 + 1) * 3 + k];
       float a2 = s_r[(ty * 4 + 2) * 3 + k];
       float a3 = s_r[(ty * 4 + 3) * 3 + k];
-      acc[0][0] = fmaf(a0, b.x, acc[0][0]); acc[0][1] = fmaf(a0, b.y, acc[0][1]);
-      acc[0][2] = fmaf(a0, b.z, acc[0][2]); acc[0][3] = fmaf(a0, b.w, acc[0][3]);
-      acc[1][0] = fmaf(a1, b.x, acc[1][0]); acc[1][1] = fmaf(a1, b.y, acc[1][1]);
-      acc[1][2] = fmaf(a1, b.z, acc[1][2]); acc[1][3] = fmaf(a1, b.w, acc[1][3]);
-      acc[2][0] = fmaf(a2, b.x, acc[2][0]); acc[2][1] = fmaf(a2, b.y, acc[2][1]);
-      acc[2][2] = fmaf(a2, b.z, acc[2][2]); acc[2][3] = fmaf(a2, b.w, acc[2][3]);
-      acc[3][0] = fmaf(a3, b.x, acc[3][0]); acc[3][1] = fmaf(a3, b.y, acc[3][1]);
-      acc[3][2] = fmaf(a3, b.z, acc[3][2]); acc[3][3] = fmaf(a3, b.w, acc[3][3]);
+      acc[0][0] = sif_mac(a0, b.x, acc[0][0]); acc[0][1] = sif_mac(a0, b.y, acc[0][1]);
+      acc[0][2] = sif_mac(a0, b.z, acc[0][2]); acc[0][3] = sif_mac(a0, b.w, acc[0][3]);
+      acc[1][0] = sif_mac(a1, b.x, acc[1][0]); acc[1][1] = sif_mac(a1, b.y, acc[1][1]);
+      acc[1][2] = sif_mac(a1, b.z, acc[1][2]); acc[1][3] = sif_mac(a1, b.w, acc[1][3]);
+      acc[2][0] = sif_mac(a2, b.x, acc[2][0]); acc[2][1] = sif_mac(a2, b.y, acc[2][1]);
+      acc[2][2] = sif_mac(a2, b.z, acc[2][2]); acc[2][3] = sif_mac(a2, b.w, acc[2][3]);
+      acc[3][0] = sif_mac(a3, b.x, acc[3][0]); acc[3][1] = sif_mac(a3, b.y, acc[3][1]);
+      acc[3][2] = sif_mac(a3, b.z, acc[3][2]); acc[3][3] = sif_mac(a3, b.w, acc[3][3]);
     }
     __syncthreads();
   }
 
-  // epilogue: Pearson, prior, per-thread best over its 4 positions for each of its 4 patches
+  // epilogue: Pearson or L2, prior, per-thread best over its 4 positions for each of its 4 patches
   const float nf = (float)kdim;
   unsigned long long best[4] = {0ull, 0ull, 0ull, 0ull};
 #pragma unroll
@@ -188,8 +234,15 @@ __global__ void __launch_bounds__(256) sif_score_simt_kernel(const float* __rest
       int j = j0 + ty * 4 + a;
       if (j >= wp) continue;
       float4 ys = reinterpret_cast<const float4*>(ystat)[((int64_t)img * hp + i) * wp + j];
-      float s = sif_pearson(acc[a][b], ys.x, ys.y, ys.z, sx, xm, denx, nf);
-      if (use_mask) s = __fmul_rn(s, sif_mask_exact(p, i, j, hh, ww, ph, PW));
+      float s;
+      if constexpr (METRIC == SIF_L2) {  // the negated masked distance: its argmax is tf.argmin's
+        s = sif_l2((float)acc[a][b], ps[1], ys.w);
+        if (use_mask) s = __fmul_rn(s, sif_mask_exact(p, i, j, hh, ww, ph, PW));
+        s = -s;
+      } else {
+        s = sif_pearson(acc[a][b], ys.x, ys.y, ys.z, sx, xm, denx, nf);
+        if (use_mask) s = __fmul_rn(s, sif_mask_exact(p, i, j, hh, ww, ph, PW));
+      }
       unsigned long long key = sif_pack(s, (unsigned)(i * wp + j));
       best[b] = key > best[b] ? key : best[b];
     }
@@ -208,7 +261,7 @@ __global__ void __launch_bounds__(256) sif_score_simt_kernel(const float* __rest
 
 __global__ void sif_finalize_keys_kernel(const unsigned long long* __restrict__ keys, int64_t np, int wp,
                                          int32_t* __restrict__ row, int32_t* __restrict__ col,
-                                         float* __restrict__ best) {
+                                         float* __restrict__ best, int negate) {
   int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= np) return;
   unsigned long long k = keys[idx];
@@ -217,7 +270,7 @@ __global__ void sif_finalize_keys_kernel(const unsigned long long* __restrict__ 
   if (k != 0ull) sif_unpack(k, &s, &pos);
   row[idx] = (int32_t)(pos / (unsigned)wp);
   col[idx] = (int32_t)(pos % (unsigned)wp);
-  if (best) best[idx] = s;
+  if (best) best[idx] = negate ? -s : s;  // L2 keys hold the negated masked distance
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -265,15 +318,14 @@ __global__ void sif_gather_kernel(const float* __restrict__ y, const int32_t* __
 // ---------------------------------------------------------------------------------------------
 // C ABI
 // ---------------------------------------------------------------------------------------------
-extern "C" {
-
-int dsin_sif_prepare(dsin_handle_t h, const float* xdec, const float* ydec, int n, int hh, int ww, int ph,
-                     int pw, float* q, float* r, float* pstat, float* ystat, void* stream) {
+template <int METRIC>
+static int sif_prepare(dsin_handle_t h, const float* xdec, const float* ydec, int n, int hh, int ww, int ph, int pw,
+                       float* q, float* r, float* pstat, float* ystat, void* stream) {
   DSIN_REQUIRE(h, xdec && ydec && q && r && pstat && ystat, "null pointer");
   DSIN_REQUIRE(h, n > 0 && ph > 1 && pw > 1 && hh % ph == 0 && ww % pw == 0, "image must tile into patches");
   cudaStream_t st = (cudaStream_t)stream;
   int64_t npix = (int64_t)n * hh * ww;
-  sif_transform_kernel<<<(unsigned)((npix + 255) / 256), 256, 0, st>>>(xdec, ydec, q, r, n, hh, ww, ph, pw);
+  sif_transform_kernel<METRIC><<<(unsigned)((npix + 255) / 256), 256, 0, st>>>(xdec, ydec, q, r, n, hh, ww, ph, pw);
   DSIN_LAUNCHED(h);
   int64_t np = (int64_t)n * (hh / ph) * (ww / pw);
   sif_patch_stats_kernel<<<(unsigned)((np * 32 + 255) / 256), 256, 0, st>>>(q, pstat, np, ph * pw * 3);
@@ -293,14 +345,10 @@ int dsin_sif_prepare(dsin_handle_t h, const float* xdec, const float* ydec, int 
   return DSIN_OK;
 }
 
-int64_t dsin_sif_workspace_bytes(int n, int hh, int ww, int ph, int pw, int method) {
-  int64_t P = (int64_t)(hh / ph) * (ww / pw);
-  return sif_tc_workspace_bytes(n, hh, ww, ph, pw, method) + n * P * 8 + 1024;
-}
-
-int dsin_sif_match(dsin_handle_t h, const float* q, const float* r, const float* pstat, const float* ystat,
-                   int n, int hh, int ww, int ph, int pw, int use_mask, int method, int32_t* row,
-                   int32_t* col, float* best, void* workspace, void* stream) {
+template <int METRIC>
+static int sif_match(dsin_handle_t h, const float* q, const float* r, const float* pstat, const float* ystat, int n,
+                     int hh, int ww, int ph, int pw, int use_mask, int method, int32_t* row, int32_t* col, float* best,
+                     void* workspace, void* stream) {
   DSIN_REQUIRE(h, q && r && pstat && ystat && row && col && workspace, "null pointer");
   DSIN_REQUIRE(h, n > 0 && hh % ph == 0 && ww % pw == 0, "image must tile into patches");
   cudaStream_t st = (cudaStream_t)stream;
@@ -312,17 +360,54 @@ int dsin_sif_match(dsin_handle_t h, const float* q, const float* r, const float*
   if (method == 0) {
     DSIN_REQUIRE(h, pw == 24, "SIMT scorer is built for 24-pixel-wide patches");
     dim3 grid((wp + 63) / 64, hp, n * ((P + 63) / 64));
-    sif_score_simt_kernel<24><<<grid, 256, 0, st>>>(q, r, pstat, ystat, n, hh, ww, ph, use_mask, keys);
+    sif_score_simt_kernel<24, METRIC><<<grid, 256, 0, st>>>(q, r, pstat, ystat, n, hh, ww, ph, use_mask, keys);
     DSIN_LAUNCHED(h);
   } else {
-    int rc = sif_tc_match(h, q, r, pstat, ystat, n, hh, ww, ph, pw, use_mask, keys,
+    int rc = sif_tc_match(h, q, r, pstat, ystat, n, hh, ww, ph, pw, use_mask, METRIC, keys,
                           (char*)workspace + sizeof(unsigned long long) * (size_t)n * P, st);
     if (rc != DSIN_OK) return rc;
   }
   int64_t np = (int64_t)n * P;
-  sif_finalize_keys_kernel<<<(unsigned)((np + 255) / 256), 256, 0, st>>>(keys, np, wp, row, col, best);
+  sif_finalize_keys_kernel<<<(unsigned)((np + 255) / 256), 256, 0, st>>>(keys, np, wp, row, col, best,
+                                                                       METRIC == SIF_L2);
   DSIN_LAUNCHED(h);
   return DSIN_OK;
+}
+
+extern "C" {
+
+int dsin_sif_prepare(dsin_handle_t h, const float* xdec, const float* ydec, int n, int hh, int ww, int ph,
+                     int pw, float* q, float* r, float* pstat, float* ystat, void* stream) {
+  return sif_prepare<SIF_PEARSON>(h, xdec, ydec, n, hh, ww, ph, pw, q, r, pstat, ystat, stream);
+}
+
+int dsin_sif_prepare_lab(dsin_handle_t h, const float* xdec, const float* ydec, int n, int hh, int ww, int ph,
+                         int pw, float* q, float* r, float* pstat, float* ystat, void* stream) {
+  return sif_prepare<SIF_L2>(h, xdec, ydec, n, hh, ww, ph, pw, q, r, pstat, ystat, stream);
+}
+
+int64_t dsin_sif_workspace_bytes(int n, int hh, int ww, int ph, int pw, int method) {
+  int64_t P = (int64_t)(hh / ph) * (ww / pw);
+  return sif_tc_workspace_bytes(n, hh, ww, ph, pw, method) + n * P * 8 + 1024;
+}
+
+int64_t dsin_sif_work_count_offset(const void* workspace, int n, int hh, int ww, int ph, int pw) {
+  const int64_t keys = (int64_t)n * (hh / ph) * (ww / pw) * 8;
+  return keys + sif_tc_work_count_offset((const char*)workspace + keys, n, hh, ww, ph, pw);
+}
+
+int dsin_sif_match(dsin_handle_t h, const float* q, const float* r, const float* pstat, const float* ystat,
+                   int n, int hh, int ww, int ph, int pw, int use_mask, int method, int32_t* row,
+                   int32_t* col, float* best, void* workspace, void* stream) {
+  return sif_match<SIF_PEARSON>(h, q, r, pstat, ystat, n, hh, ww, ph, pw, use_mask, method, row, col, best,
+                                workspace, stream);
+}
+
+int dsin_sif_match_l2(dsin_handle_t h, const float* q, const float* r, const float* pstat, const float* ystat,
+                      int n, int hh, int ww, int ph, int pw, int use_mask, int method, int32_t* row,
+                      int32_t* col, float* best, void* workspace, void* stream) {
+  return sif_match<SIF_L2>(h, q, r, pstat, ystat, n, hh, ww, ph, pw, use_mask, method, row, col, best, workspace,
+                           stream);
 }
 
 int dsin_sif_gather(dsin_handle_t h, const float* y, const int32_t* row, const int32_t* col, int n, int hh,

@@ -389,7 +389,8 @@ def probclass_bits_tc(qbar_nchw, symbols, pctc, pad_value, terms=3, want_bits=Tr
     return bits, sums
 
 
-def sif_prepare(xdec_nhwc, ydec_nhwc, ph, pw):
+def sif_prepare(xdec_nhwc, ydec_nhwc, ph, pw, lab=False):
+    """Pearson: normalised H1/H2/H3 transform; lab=True: CIELAB of the raw pixels (dsin_sif_prepare_lab)."""
     h = handle()
     n, hh, ww, _ = xdec_nhwc.shape
     dev = xdec_nhwc.device
@@ -398,27 +399,51 @@ def sif_prepare(xdec_nhwc, ydec_nhwc, ph, pw):
     r = torch.empty((n, hh, ww, 3), dtype=torch.float32, device=dev)
     pstat = torch.empty((n, P, 4), dtype=torch.float32, device=dev)
     ystat = torch.empty((n, hh - ph + 1, ww - pw + 1, 4), dtype=torch.float32, device=dev)
-    h.check(h.lib.dsin_sif_prepare(h.ptr, _p(_chk(xdec_nhwc)), _p(_chk(ydec_nhwc)), n, hh, ww, ph, pw, _p(q), _p(r),
-                                   _p(pstat), _p(ystat), _stream()))
+    fn = h.lib.dsin_sif_prepare_lab if lab else h.lib.dsin_sif_prepare
+    h.check(fn(h.ptr, _p(_chk(xdec_nhwc)), _p(_chk(ydec_nhwc)), n, hh, ww, ph, pw, _p(q), _p(r), _p(pstat), _p(ystat),
+               _stream()))
     return q, r, pstat, ystat
 
 
-def sif_match(q, r, pstat, ystat, ph, pw, use_mask=True, method=0):
+def sif_prepare_lab(xdec_nhwc, ydec_nhwc, ph, pw):
+    return sif_prepare(xdec_nhwc, ydec_nhwc, ph, pw, lab=True)
+
+
+def sif_match(q, r, pstat, ystat, ph, pw, use_mask=True, method=0, l2=False, work=None):
+    """Pearson: argmax of the masked correlation; l2=True: argmin of the masked L2 distance (dsin_sif_match_l2), best
+    is then the masked distance at the argmin.  work: optional uint8 workspace of sif_workspace_bytes (read it back
+    with sif_work_count)."""
     h = handle()
     n, hh, ww, _ = r.shape
     P = q.shape[1]
     dev = r.device
-    ws = int(h.lib.dsin_sif_workspace_bytes(n, hh, ww, ph, pw, method))
-    work = torch.empty(ws, dtype=torch.uint8, device=dev)
+    if work is None:
+        work = torch.empty(sif_workspace_bytes(n, hh, ww, ph, pw, method), dtype=torch.uint8, device=dev)
+    assert work.dtype == torch.uint8 and work.numel() >= sif_workspace_bytes(n, hh, ww, ph, pw, method)
     row = torch.empty((n, P), dtype=torch.int32, device=dev)
     col = torch.empty((n, P), dtype=torch.int32, device=dev)
     best = torch.empty((n, P), dtype=torch.float32, device=dev)
+    fn = h.lib.dsin_sif_match_l2 if l2 else h.lib.dsin_sif_match
     e0 = PROF.begin()
-    h.check(h.lib.dsin_sif_match(h.ptr, _p(_chk(q)), _p(_chk(r)), _p(_chk(pstat)), _p(_chk(ystat)), n, hh, ww, ph, pw,
-                                 int(use_mask), int(method), _p(row), _p(col), _p(best), _p(work), _stream()))
+    h.check(fn(h.ptr, _p(_chk(q)), _p(_chk(r)), _p(_chk(pstat)), _p(_chk(ystat)), n, hh, ww, ph, pw, int(use_mask),
+               int(method), _p(row), _p(col), _p(best), _p(work), _stream()))
     if e0 is not None:
-        PROF.end(e0, "sif_match", 2.0 * n * (hh - ph + 1) * (ww - pw + 1) * P * (ph * pw * 3))
+        PROF.end(e0, "sif_match_l2" if l2 else "sif_match", 2.0 * n * (hh - ph + 1) * (ww - pw + 1) * P * (ph * pw * 3))
     return row, col, best
+
+
+def sif_match_l2(q, r, pstat, ystat, ph, pw, use_mask=True, method=0, work=None):
+    return sif_match(q, r, pstat, ystat, ph, pw, use_mask=use_mask, method=method, l2=True, work=work)
+
+
+def sif_workspace_bytes(n, hh, ww, ph, pw, method):
+    return int(handle().lib.dsin_sif_workspace_bytes(n, hh, ww, ph, pw, method))
+
+
+def sif_work_count(work, n, hh, ww, ph, pw):
+    """Number of (patch, group) work items the last method-1 sif_match on `work` rescored exhaustively."""
+    off = int(handle().lib.dsin_sif_work_count_offset(_p(work), n, hh, ww, ph, pw))
+    return int(work[off:off + 4].view(torch.int32).item())
 
 
 def sif_gather(y_nhwc, row, col, ph, pw):

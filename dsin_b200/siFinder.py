@@ -1,9 +1,21 @@
-"""SI-Finder on libdsin_b200 (/root/reference/src/siFinder.py:7-53, Pearson branch).
+"""SI-Finder on libdsin_b200 (/root/reference/src/siFinder.py:7-53).
 
 ``siFinder(x_patches, y_images, mask, batch_size, ph, pw, H, W, ae_config, y_dec)`` keeps the
 reference signature (channel-last tensors).  ``match_images`` is the whole-image entry used
 by SI_full_img: it never tiles x into patches on the host and never materialises the
 correlation map (``ncc`` is returned as None).
+
+Both matching modes of the reference are built, selected by ``ae_config.use_L2andLAB`` as there:
+
+* False (the shipped config): the images are normalised and mapped to H1/H2/H3, windows are scored by
+  Pearson correlation times the Gaussian prior, and the argmax is taken.
+* True: the RAW 0..255 pixels are mapped to CIELAB (rgb_to_lab assumes sRGB in [0, 1], so the values come out
+  far outside the usual LAB ranges: white has L ~ 9342), windows are scored by the squared L2 distance
+  ``(sum_x_square - 2 * xy) + sum_y_square`` times the prior, and the argMIN is taken (first index on ties).
+  ``q`` / ``r`` are then the LAB images, ``extremum`` the argmin index and ``best`` the masked distance there.
+  Quirk kept from the reference: the prior, a factor in (0, 1] that is largest at the patch's own position,
+  MULTIPLIES a distance here, so it makes far-away windows cheaper and pulls the matches toward the image
+  corners rather than toward the patch (use_gauss_mask = False avoids it).
 """
 from __future__ import annotations
 
@@ -11,7 +23,7 @@ import torch
 
 from . import ops
 
-METHOD = 1  # 0: fp32 SIMT scorer (cross-check); 1: tcgen05 coarse scorer + exact rescoring
+METHOD = 1  # 0: SIMT scorer (cross-check); 1: tcgen05 coarse scorer + exact rescoring
 
 
 class GaussianPrior(object):
@@ -22,11 +34,15 @@ class GaussianPrior(object):
         self.H, self.W, self.ph, self.pw = H, W, ph, pw
 
 
+def uses_l2(ae_config):
+    """The matching mode ae_config selects: True for L2 + LAB (use_L2andLAB), False for Pearson."""
+    return bool(ae_config is not None and getattr(ae_config, "use_L2andLAB", False))
+
+
 def match_images(x_dec_nhwc, y_nhwc, y_dec_nhwc, ph, pw, use_mask, ae_config=None):
-    if ae_config is not None and getattr(ae_config, "use_L2andLAB", False):
-        raise NotImplementedError("the L2+LAB variant is disabled in the shipped config and not built")
-    q, r, pstat, ystat = ops.sif_prepare(x_dec_nhwc, y_dec_nhwc, ph, pw)
-    row, col, best = ops.sif_match(q, r, pstat, ystat, ph, pw, use_mask=use_mask, method=METHOD)
+    l2 = uses_l2(ae_config)
+    q, r, pstat, ystat = ops.sif_prepare(x_dec_nhwc, y_dec_nhwc, ph, pw, lab=l2)
+    row, col, best = ops.sif_match(q, r, pstat, ystat, ph, pw, use_mask=use_mask, method=METHOD, l2=l2)
     y_syn = ops.sif_gather(y_nhwc, row, col, ph, pw)
     return y_syn, q, r, row, col, best
 

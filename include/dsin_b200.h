@@ -201,6 +201,23 @@ int dsin_sif_match(dsin_handle_t h, const float* q, const float* r, const float*
                    const float* ystat, int n, int hh, int ww, int ph, int pw, int use_mask,
                    int method, int32_t* row, int32_t* col, float* best, void* workspace,
                    void* stream);
+/* L2 + LAB matching (ae_config.use_L2andLAB = True), same arguments as the two entry points above.
+ * dsin_sif_prepare_lab replaces rgb_transform's LAB branch, rgb_to_lab (src/siFinder.py:13-17,145-146,157-195):
+ *    q, r are CIELAB transforms of the RAW 0..255 pixels (no normalisation); pstat, ystat as above.
+ * dsin_sif_match_l2 replaces L2_or_pearson_corr's L2 branch, the mask multiply and tf.argmin
+ *    (src/siFinder.py:20,28-29,91-103): argmin over positions of ((sx2 - 2*xy) + sy2) * mask_p, first index on
+ *    ties -> row, col; best = the masked distance at the argmin.  Inputs must lie in [0, 255] (|LAB| < 65504 for
+ *    the fp16 coarse pass of method 1).                                                                      */
+int dsin_sif_prepare_lab(dsin_handle_t h, const float* xdec_nhwc, const float* ydec_nhwc, int n, int hh,
+                         int ww, int ph, int pw, float* q, float* r, float* pstat, float* ystat,
+                         void* stream);
+int dsin_sif_match_l2(dsin_handle_t h, const float* q, const float* r, const float* pstat,
+                      const float* ystat, int n, int hh, int ww, int ph, int pw, int use_mask,
+                      int method, int32_t* row, int32_t* col, float* best, void* workspace,
+                      void* stream);
+/* Byte offset, within the workspace of a method-1 dsin_sif_match / dsin_sif_match_l2 call, of the int32 number
+ * of (patch, group) work items that the exact pass rescored exhaustively (diagnostics).                        */
+int64_t dsin_sif_work_count_offset(const void* workspace, int n, int hh, int ww, int ph, int pw);
 int dsin_sif_gather(dsin_handle_t h, const float* y_nhwc, const int32_t* row, const int32_t* col,
                     int n, int hh, int ww, int ph, int pw, float* ysyn_nhwc, void* stream);
 
