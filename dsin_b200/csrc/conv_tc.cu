@@ -600,33 +600,16 @@ extern "C" int dsin_conv2d_tc(dsin_handle_t h, const dsin_conv_desc_t* d, int te
     p.tiles_w = (p.GW + BW - 1) / BW; p.tiles_h = (p.GH + BH - 1) / BH;
     p.total_tiles = d->n * p.tiles_w * p.tiles_h;
     if (!(d->flags & (DSIN_CONV_NO_HALO | DSIN_CONV_PAIR_SHARED)) && k == 3 && d->stride == 1 && d->cin == 32 &&
-        d->cout == 32 && d->dilation >= 1 && d->dilation <= 4 && dil_x == d->dilation && y_hi && !y_f32 && !res1_hi &&
-        !res2_hi && d->post == DSIN_POST_NONE && (terms == 1 || y_lo)) {
-      // 32-channel layer with a small dilation: halo-tile kernel with a resident filter (conv_h32.cu)
-      ConvH32Args q;
-      memset(&q, 0, sizeof(q));
-      q.scale = scale; q.shift = shift;
-      q.yh = (__half*)y_hi; q.yl = (__half*)y_lo;
-      q.n_out = d->n; q.OH = p.OH; q.OW = p.OW; q.cout = 32; q.act = d->act; q.terms = terms;
-      q.ntaps = 9;
-      for (int t = 0; t < 9; ++t) {
-        q.tz[t] = 0; q.ty[t] = (short)((t / 3) * d->dilation); q.tx[t] = (short)((t % 3) * d->dilation); q.tw[t] = (short)t;
-      }
-      q.hw = 8 + 2 * d->dilation; q.hh = 16 + 2 * d->dilation; q.hd = 1;
-      q.ox = -d->dilation; q.oy = -d->dilation;
-      const int rc = conv_h32_launch(h, (const __half*)x_hi, (const __half*)x_lo, (const __half*)w_hi,
-                                     (const __half*)w_lo, d->w, d->h, d->n, 9, q, st);
-      if (rc != DSIN_ERR_UNSUPPORTED) return rc;
-    }
-    if (!(d->flags & (DSIN_CONV_NO_HALO | DSIN_CONV_PAIR_SHARED)) && k == 3 && d->stride == 1 && d->cin == 32 &&
-        d->cout == 32 && d->dilation > 4 && dil_x == d->dilation && y_hi && !y_f32 && !res1_hi && !res2_hi &&
+        d->cout == 32 && d->dilation >= 1 && dil_x == d->dilation && y_hi && !y_f32 && !res1_hi && !res2_hi &&
         d->post == DSIN_POST_NONE && (terms == 1 || y_lo)) {
-      // 32-channel layer with a large dilation: row-band kernel (conv_dil.cu)
+      // 32-channel layer (the SI-Net's 3x3 layers, every dilation): row-band kernel (conv_dil.cu).  At dilation 1, 2, 4
+      // it also beats the halo-tile kernel (conv_h32.cu, which keeps the probability model's layers), see DESIGN 5.2
       ConvDilArgs q;
       memset(&q, 0, sizeof(q));
       q.scale = scale; q.shift = shift;
       q.yh = (__half*)y_hi; q.yl = (__half*)y_lo;
       q.n = d->n; q.H = d->h; q.W = d->w; q.dil = d->dilation; q.act = d->act; q.terms = terms;
+      q.ksteps = (d->flags & DSIN_CONV_CIN16) ? 1 : 2;
       const int rc = conv_dil_launch(h, (const __half*)x_hi, (const __half*)x_lo, (const __half*)w_hi,
                                      (const __half*)w_lo, q, st);
       if (rc != DSIN_ERR_UNSUPPORTED) return rc;

@@ -80,12 +80,13 @@ struct ConvH32Args {
   int ox, oy;        // halo origin relative to the tile origin (-dilation for SAME, 0 for VALID)
   int tiles_w, tiles_h, total_tiles, w_plane, w_region, a_plane, na;  // filled by conv_h32_launch
 };
-// conv_dil.cu: 3x3, 32 -> 32 channels, stride 1, SAME, dilation `dil` >= 1 (meant for >= 8), split-fp16 or fp16 output
+// conv_dil.cu: 3x3, 32 -> 32 channels, stride 1, SAME, dilation `dil` >= 1, split-fp16 or fp16 output
 struct ConvDilArgs {
   const float* scale;
   const float* shift;
   __half *yh, *yl;  // output planes (n, H, W, 32); yl may be NULL with terms == 1
   int n, H, W, dil, act, terms;
+  int ksteps;       // 16-channel K-steps that carry data: 2, or 1 when input channels 16..31 are zero
   // filled by conv_dil_launch
   int nbox, bw, a_plane, w_region, nb, tiles_w, phases, seg, nseg, total_units;
 };

@@ -133,6 +133,16 @@ __device__ __forceinline__ void tmem_ld_32x16(uint32_t taddr, uint32_t (&v)[16])
       : "memory");
 }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+// the reverse of tmem_ld_32x16: thread i of the warp writes lane (base_lane + i), 16 consecutive columns
+__device__ __forceinline__ void tmem_st_32x16(uint32_t taddr, const uint32_t (&v)[16]) {
+  asm volatile(
+      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
+      "{%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};" ::"r"(taddr),
+      "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), "r"(v[8]), "r"(v[9]),
+      "r"(v[10]), "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15])
+      : "memory");
+}
+__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
 // ------------------------------------------------------------------ coalesced epilogues: staging + TMA store
 // (an accumulator row is a pixel, so direct 16-byte global accesses of a warp touch 32 different 128-byte lines;

@@ -225,6 +225,7 @@ CONV_PAIR_SHARED = 1
 CONV_NO_CTA_PAIR = 2             # cross-check: one-CTA kernel for a 128->128 layer
 CONV_NO_WEIGHT_STATIONARY = 4    # cross-check: tap-streaming CTA-pair kernel for a terms = 1 trunk layer
 CONV_NO_HALO = 8                 # cross-check: tap-streaming CTA-pair kernel for a terms = 3 trunk layer
+CONV_CIN16 = 16                  # 32->32 layer whose input channels 16..31 are zero: skip their K-step
 
 
 class _PairDesc(object):

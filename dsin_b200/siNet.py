@@ -12,10 +12,11 @@ import torch
 
 from . import ops, synth
 
-# Layer forms (all tcgen05).  Dilation <= HALO_MAX_RATE: halo-tile kernel (csrc/conv_h32.cu); larger dilations: row-band
-# kernel (csrc/conv_dil.cu) when BAND, else the tap-streaming kernel (csrc/conv_tc.cu) in the pixel-pair view (PAIR:
-# 128-byte TMA rows; PAIR_SHARED: even dilations reuse the plain 32x32 slab for both pixels of a pair).  Module
-# attributes so that tests can compare the forms against each other; the product never changes them.
+# Layer forms (all tcgen05).  Every 3x3 layer runs on the row-band kernel (csrc/conv_dil.cu); it beats the halo-tile
+# kernel (csrc/conv_h32.cu) at dilation 1, 2 and 4 too.  With BAND off, the layers with a dilation above HALO_MAX_RATE
+# run on the tap-streaming kernel (csrc/conv_tc.cu) in the pixel-pair view instead (PAIR: 128-byte TMA rows;
+# PAIR_SHARED: even dilations reuse the plain 32x32 slab for both pixels of a pair), the others stay on the band
+# kernel.  Module attributes so that tests can compare the forms against each other; the product never changes them.
 BAND = True
 PAIR = True
 PAIR_SHARED = True
@@ -52,6 +53,7 @@ class SiNet(object):
         w1[:, :, :6, :] = W[S + "g_conv1/weights"]
         self._first_padded = ops.ConvLayer(w1, None, W[S + "g_conv1/biases"], dilation=1, act=ops.ACT_LRELU02,
                                            device=self.device)
+        self._first_padded.flags = ops.CONV_CIN16  # channels 6..31 of its input are zero
         self._tc_first = None
         # the pixel-pair form of the nine 3x3 layers (only used with BAND = False, see _pair_form) is built on demand
         self._w1_padded, self._variables = w1, W
@@ -97,8 +99,7 @@ class SiNet(object):
             self._tc_first = ops.ConvTC(self._first_padded)
         use_pair = PAIR and ww % 2 == 0 and ww // 2 >= 16
         for li, tcl in enumerate([self._tc_first] + self._tc[:-1]):
-            # dilation <= 4: the plain 32-channel layer runs on the halo-tile kernel (csrc/conv_h32.cu); larger
-            # dilations on the row-band kernel (csrc/conv_dil.cu) -- both chosen by dsin_conv2d_tc from the geometry
+            # the plain 32-channel layer runs on the row-band kernel (csrc/conv_dil.cu), chosen by dsin_conv2d_tc
             if not BAND and use_pair and self.RATES[li] > HALO_MAX_RATE:
                 key = (li, PAIR_SHARED)
                 if key not in self._pair_tc:

@@ -84,9 +84,11 @@ enum { DSIN_CONV_PAIR_SHARED = 1,
        DSIN_CONV_NO_CTA_PAIR = 2, /* run a 128->128 layer on the one-CTA kernel (cross-check of the CTA-pair kernels) */
        DSIN_CONV_NO_WEIGHT_STATIONARY = 4, /* terms = 1, 3x3 128->128: use the tap-streaming CTA-pair kernel instead of
                                                the weight-stationary halo-tile kernel (cross-check) */
-       DSIN_CONV_NO_HALO = 8 /* use the tap-streaming kernels (cross-check) instead of the halo-tile kernel of the
-                                3x3 128->128 layers with terms = 3 (conv_h3) and of the halo-tile / row-band kernels of
-                                the 3x3 32->32 layers (conv_h32: dilation <= 4, conv_dil: larger dilations) */
+       DSIN_CONV_NO_HALO = 8, /* use the tap-streaming kernels (cross-check) instead of the halo-tile kernel of the
+                                3x3 128->128 layers with terms = 3 (conv_h3) and of the row-band kernel of the 3x3
+                                32->32 layers (conv_dil) */
+       DSIN_CONV_CIN16 = 16 /* 3x3 32->32 layers on the row-band kernel: input channels 16..31 are zero (the SI-Net's
+                               first layer, 6 live channels padded to 32), so their K-step is skipped */
 };
 int dsin_conv2d(dsin_handle_t h, const dsin_conv_desc_t* d, const float* x, const float* w,
                 const float* scale, const float* shift, const float* res1, const float* res2,
@@ -116,7 +118,7 @@ int dsin_conv3x3_c128_tc(dsin_handle_t h, int n, int hh, int ww, const uint16_t*
  * power-of-two factors the caller divides out of `scale`.
  * The entry point picks the kernel from the geometry: 3x3 128->128 stride 1 -> CTA-pair kernels with a halo-resident
  * activation tile (terms 3: conv_h3.cu; terms 1: weight-stationary conv_ws.cu); 3x3 32->32 stride 1 without residuals ->
- * halo tiles (dilation <= 4, conv_h32.cu) or row bands (dilation > 4, conv_dil.cu); everything else -> the
+ * row bands (any dilation, conv_dil.cu); everything else -> the
  * tap-streaming kernels (conv_tc2.cu for 128-channel outputs on CTA pairs, conv_tc.cu otherwise).  `flags` force
  * the tap-streaming forms for cross-checks. */
 int dsin_conv_tc_npad(int cout);

@@ -1,11 +1,25 @@
-"""A/B timing of the SI-Net (src/siNet.py:29-41) at batch B on one box: row-band kernel for the large dilations
-(siNet.BAND, default) vs the tap-streaming pixel-pair form, both orders; prints ms per SI-Net pass and per layer."""
+"""Timing of the SI-Net (src/siNet.py:29-41) on 320x1224 images at batch B on one box: ms per SI-Net pass, then ms per
+3x3 layer for all nine layers (by dilation) as the dispatch runs them, one JSON line each.  The first layer is timed
+on an input with 6 live channels, as in the network.
+
+    python tools/sinet_bench.py [--batch 32] [--reps 20] [--root DIR] [--label NAME]
+
+--root times the package of another tree (for example a checkout of an earlier commit with its library built) with
+this same script, so that two builds can be compared line for line on one box."""
+import argparse
+import json
 import os
 import sys
 
 import torch
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+p = argparse.ArgumentParser()
+p.add_argument("--batch", type=int, default=32)
+p.add_argument("--reps", type=int, default=20)
+p.add_argument("--root", default=os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+p.add_argument("--label", default="")
+args = p.parse_args()
+ROOT = os.path.abspath(args.root)
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -13,44 +27,42 @@ from parity_utils import make_ae  # noqa: E402
 from dsin_b200 import ops, siNet as sn, synth  # noqa: E402
 
 
+def timed(fn, reps):
+    for _ in range(3):
+        fn()
+    torch.cuda.synchronize()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    for _ in range(reps):
+        fn()
+    e1.record()
+    torch.cuda.synchronize()
+    return e0.elapsed_time(e1) / reps
+
+
 def main():
-    B = int(sys.argv[1]) if len(sys.argv) > 1 else 8
-    reps = int(sys.argv[2]) if len(sys.argv) > 2 else 30
-    H, W = 320, 1224
+    B, H, W = args.batch, 320, 1224
+    dev = torch.cuda.get_device_properties(0)
+    common = {"label": args.label, "root": os.path.basename(ROOT), "gpu": dev.name, "batch": B, "hw": [H, W]}
     ae = make_ae(H, W, synth.make_weights(0, residual_gamma=0.25))
     a = torch.rand(B, H, W, 3, device="cuda") * 255
     b = torch.rand(B, H, W, 3, device="cuda") * 255
-    outs = {}
-    for band in (True, False, False, True):
-        sn.BAND = band
-        for _ in range(3):
-            y = ae._siNet.fused(a, b, terms=3)
-        torch.cuda.synchronize()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        for _ in range(reps):
-            y = ae._siNet.fused(a, b, terms=3)
-        e1.record()
-        torch.cuda.synchronize()
-        outs[band] = y._dsin_nhwc.clone()
-        print("BAND=%s: %.3f ms per SI-Net pass at batch %d" % (band, e0.elapsed_time(e1) / reps, B), flush=True)
-    print("max |band - pair| = %.3e grey levels" % float((outs[True] - outs[False]).abs().max()))
-    # per layer
-    cur = ops.f32_to_split(torch.randn(B, H, W, 32, device="cuda"))
-    for li in (3, 4, 5, 6, 7):
-        rate = sn.SiNet.RATES[li]
-        tcl = ae._siNet._tc[li - 1]
-        for name, flags in (("band", 0), ("stream", ops.CONV_NO_HALO)):
-            for _ in range(2):
-                ops.conv_tc(cur, tcl, terms=3, flags=flags)
-            torch.cuda.synchronize()
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record()
-            for _ in range(reps):
-                ops.conv_tc(cur, tcl, terms=3, flags=flags)
-            e1.record()
-            torch.cuda.synchronize()
-            print("  rate %3d %-6s %.3f ms" % (rate, name, e0.elapsed_time(e1) / reps), flush=True)
+    ms = timed(lambda: ae._siNet.fused(a, b, terms=3), args.reps)
+    print(json.dumps(dict(common, what="sinet_pass", ms=round(ms, 4), ms_per_pair=round(ms / B, 5))), flush=True)
+    net = ae._siNet
+    x = torch.randn(B, H, W, 32, device="cuda")
+    x6 = x.clone()
+    x6[..., 6:] = 0
+    cur, cur6 = ops.f32_to_split(x), ops.f32_to_split(x6)
+    total = 0.0
+    for li, rate in enumerate(sn.SiNet.RATES):
+        tcl = net._tc_first if li == 0 else net._tc[li - 1]
+        inp = cur6 if li == 0 else cur
+        ms = timed(lambda: ops.conv_tc(inp, tcl, terms=3), args.reps)
+        total += ms
+        print(json.dumps(dict(common, what="layer", layer=li + 1, dilation=rate, ms=round(ms, 4),
+                              ms_per_pair=round(ms / B, 5))), flush=True)
+    print(json.dumps(dict(common, what="nine_layers", ms=round(total, 4), ms_per_pair=round(total / B, 5))), flush=True)
 
 
 if __name__ == "__main__":
